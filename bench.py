@@ -2,7 +2,7 @@
 """bench.py -- the north-star measurement: RWKV-6-World-7B-shape Q5_1, single-token decode and 128-token
 prefill through the rwkv.h C ABI of rwkv.cpp_b200/librwkv.so, on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload rwkv6-7b:Q5_1]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload rwkv6-7b:Q5_1] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one single-token evaluation (with logits) of the whole model. Prints ONE JSON line:
@@ -50,6 +50,8 @@ def parse_args():
     ap.add_argument("--cpu-budget-s", type=float, default=20.0, help="CPU seconds the bounded reference sample may take per leg")
     ap.add_argument("--mode", default="decode", choices=["decode", "prefill"],
                     help="headline metric: single-token decode tokens/s (default) or 128-token-chunk prefill tokens/s (one step = one chunk)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps of the headline metric, write the logits and recurrent state of its last step as DIR/<name>.npy (float32)")
     # internal: the reference library only ever runs in child processes (hard timeouts), see cpu_reference_leg
     ap.add_argument("--ref-child", default=None, choices=["probe", "full"], help=argparse.SUPPRESS)
     ap.add_argument("--ref-threads", default="8", help=argparse.SUPPRESS)
@@ -125,6 +127,25 @@ def host_buffers(n_state, n_logits, kind="pinned"):
             pass
     s, l = np.zeros(n_state, np.float32), np.zeros(n_logits, np.float32)
     return s, l, s.ctypes.data, l.ctypes.data, "pageable"
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(L, ctx, n_state, n_vocab, out_dir):
+    """Writes what the last resident step left on the device, the arrays a caller of rwkv_b200_eval_resident reads back: the logits
+    of its last token and the recurrent state. The inputs are seeded, so two builds run with the same arguments can be compared
+    array by array. A state too large for the 64 MB budget is written as a fixed sample (seed 0, ascending indices)."""
+    logits, state = np.zeros(n_vocab, np.float32), np.zeros(n_state, np.float32)
+    ok = L.rwkv_b200_stage_logits(ctx.ptr, logits.ctypes.data_as(PF), None) and L.rwkv_b200_state_store(ctx.ptr, state.ctypes.data_as(PF))
+    assert ok, "reading the outputs of the last step back failed"
+    room = (DUMP_BYTES - logits.nbytes - 2 * 4096) // state.itemsize       # 4 KB per .npy header is ample
+    if state.size > room:
+        state = state[np.sort(np.random.default_rng(0).choice(state.size, room, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), logits)
+    np.save(os.path.join(out_dir, "state.npy"), state)
+    log("outputs of the last timed step written to %s (logits %d, state %d of %d values)" % (out_dir, logits.size, state.size, n_state))
 
 
 def prefill_matmul_flops(preset, n_tokens):
@@ -489,6 +510,8 @@ def run_ours(args, rank, world, dist):
     windows.append((w0, time.time()))
     decode_launches = (L.rwkv_b200_kernel_launch_count() - launches0) * KD // (KD + W)
     assert ms > 0, "device timing failed"
+    if args.dump_outputs and not prefill_mode:
+        dump_outputs(L, ctx, n_state, n_vocab, args.dump_outputs)
     ms_max = max_over_ranks(ms)
     decode_tps = world * KD / (ms_max / 1e3)
     step_ms = ms_max / KD
@@ -532,6 +555,8 @@ def run_ours(args, rank, world, dist):
     w0 = time.time()
     pms = L.rwkv_b200_time_resident(ctx.ptr, tok_arr, PREFILL_TOKENS, P, W if prefill_mode else 2, True)
     windows.append((w0, time.time()))
+    if args.dump_outputs and prefill_mode:
+        dump_outputs(L, ctx, n_state, n_vocab, args.dump_outputs)
     prefill_launches = (L.rwkv_b200_kernel_launch_count() - launches0) * P // (P + (W if prefill_mode else 2))
     arr128 = (ctypes.c_uint32 * PREFILL_TOKENS)(*toks[:PREFILL_TOKENS])
     reps = P if prefill_mode else max(2, P // 2)
@@ -835,6 +860,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     dist = None
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        raise SystemExit("--dump-outputs writes the outputs of this library's one-process run (--impl ours, one GPU)")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
